@@ -32,6 +32,7 @@ FIRST_SEED = 100000          # utterance i of the workload = synth_utt(FIRST_SEE
 STRONG_UTTS = 888            # fixed list of the strong-scaling side measurement (utterances 0..887 of the job)
 MMA_FLOOR_CYCLES = 86.4      # measured: cycles per 128 x N x 16 kind::f16 MMA fed from shared memory, N <= 128
                              # (tools/tc/tc_chain_probe.cu, profiles/r2_tc_chain_probe_uniform_issue.txt)
+DUMP_LIMIT_BYTES = 64 << 20  # --dump-outputs writes at most this much
 
 
 def synth_batch(first_seed, n_utt, pinned=False):
@@ -324,7 +325,7 @@ def partition_secondary(api_model, iargs, rank, world, torch, dist, barrier):
 
 def _ref_worker(job):
   """One process of the CPU legs: decodes the first `n_frames` frames of workload utterance `seed` with the
-  unmodified reference (kind 'reference': baseline/_ref through its public predict()), the reference on a CUDA
+  unmodified reference (kind 'reference': oracle/_ref through its public predict()), the reference on a CUDA
   device ('reference_cuda') or the oracle port; returns (seconds, labels)."""
   kind, weights_path, seed, n_frames, threads = job
   import torch
@@ -333,9 +334,9 @@ def _ref_worker(job):
   from uisrnn_b200.synth import synth_utt
   x = synth_utt(seed, n_frames=N_FRAMES, dim=DIM)[0][:n_frames]
   if kind in ('reference', 'reference_cuda'):
-    sys.path[:0] = [os.path.join(ROOT, 'oracle', 'shims'), os.path.join(ROOT, 'baseline', '_ref')]
+    sys.path[:0] = [os.path.join(ROOT, 'oracle', 'shims'), os.path.join(ROOT, 'oracle', '_ref')]
     import uisrnn as ref
-    assert 'baseline' in ref.__file__
+    assert os.path.join('oracle', '_ref') in ref.__file__
     argv, sys.argv = sys.argv, [sys.argv[0]]
     try:
       margs, _, iargs = ref.parse_arguments()
@@ -372,7 +373,7 @@ def _ref_worker(job):
 
 
 def have_reference():
-  return os.path.exists(os.path.join(ROOT, 'baseline', '_ref', 'uisrnn', 'uisrnn.py'))
+  return os.path.exists(os.path.join(ROOT, 'oracle', '_ref', 'uisrnn', 'uisrnn.py'))
 
 
 def run_in_fresh_process(jobs, procs=1):
@@ -384,7 +385,7 @@ def run_in_fresh_process(jobs, procs=1):
 
 def cpu_baseline_and_parity(gpu_labels_of):
   """(a) cpu_baseline: SURVEY 8(d)(i), the unmodified reference in ONE process with the default torch threads on a
-  bounded sample (2 slices x 40 frames of workload utterances; the oracle port if baseline/_ref is absent);
+  bounded sample (2 slices x 40 frames of workload utterances; the oracle port if oracle/_ref is absent);
   (b) parity: full 500-frame utterances of the timed batch decoded by the oracle port -- the checker -- and compared
   with the labels the GPU produced for the same utterances."""
   import torch
@@ -402,7 +403,7 @@ def cpu_baseline_and_parity(gpu_labels_of):
          'sample': '%d slice x %d frames of a workload utterance (seed %d), one process, %d torch threads (default %d, '
                    'usable cores %d), %s; %.1f s in predict(), %.1f s with start-up' % (
                        n_slices, slice_frames, FIRST_SEED, threads, torch.get_num_threads(), host_info()['usable_cores'],
-                       'unmodified reference predict() from baseline/_ref' if kind == 'reference' else 'oracle/uis_oracle.py port',
+                       'unmodified reference predict() from oracle/_ref' if kind == 'reference' else 'oracle/uis_oracle.py port',
                        busy, wall)}
   # parity: utterances of the batch at their whole length (the reference-decoded ones are checked separately)
   which = sorted(gpu_labels_of.keys())
@@ -448,7 +449,7 @@ def run_reference(args):
   value = frames * len(times) / total
   sample = ('%d processes x 1 utterance slice of %d frames per step (the workload generator and seeds of the GPU arm), '
             '%s, 1 torch thread per process; calibration step with 16-frame slices: %.1f s' % (
-                procs, n_frames, 'unmodified reference predict() from baseline/_ref' if kind == 'reference'
+                procs, n_frames, 'unmodified reference predict() from oracle/_ref' if kind == 'reference'
                 else 'oracle/uis_oracle.py port', t16))
   secondary = {}
   try:  # SURVEY 8(d)(i): one process, default torch threads
@@ -481,6 +482,21 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------- this repo's arm
+
+def dump_outputs(path, out):
+  """Writes the labels the timed path returned in its last step, one row per utterance of the job's list, as float32 to
+  PATH/labels.npy, and the list index of each row to PATH/labels_utterances.npy (utterance i is synth_utt(FIRST_SEED
+  + i), so two builds run with the same arguments can be compared output for output).  Where all rows would exceed
+  DUMP_LIMIT_BYTES, a fixed seeded sample of the rows is written."""
+  labels = np.asarray([np.asarray(o) for o in out], dtype=np.float32)
+  rows = np.arange(len(labels))
+  cap = (DUMP_LIMIT_BYTES - 4096) // (labels.shape[1] * 4 + 8)   # 4096: room for the two .npy headers
+  if len(rows) > cap:
+    rows = np.sort(np.random.default_rng(0).choice(len(rows), cap, replace=False))
+  os.makedirs(path, exist_ok=True)
+  np.save(os.path.join(path, 'labels.npy'), labels[rows])
+  np.save(os.path.join(path, 'labels_utterances.npy'), rows.astype(np.float64))
+
 
 def build_api_model(weights, local, torch):
   import uisrnn
@@ -610,6 +626,8 @@ def run_b200(args):
     if world > 1:
       dist.destroy_process_group()
     return
+  if args.dump_outputs:  # rank 0 holds the whole ordered result of the e2e leg, equal to the device-resident one
+    dump_outputs(args.dump_outputs, out)
 
   # labels of the utterances the unmodified reference decoded (tests/golden/synth500_bench.npz): whichever rank
   # owned them, the merged result of the partitioned run must reproduce them
@@ -742,7 +760,13 @@ def main():
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--pageable', action='store_true', help='e2e leg from ordinary (pageable) numpy arrays instead of pinned ones')
   ap.add_argument('--no-secondary', action='store_true', help='skip the config-3 / config-4 side measurements')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='after the timed steps, write the labels of the last step to DIR/*.npy (e.g. bench_outputs/)')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs applies to --impl b200 (the reference arm decodes slices sized by a timing calibration)')
   if args.impl == 'reference':
     run_reference(args)
   else:

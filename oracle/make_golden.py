@@ -1,9 +1,9 @@
 #!/usr/bin/env python3
 """Generate the golden fixtures under tests/golden/ by RUNNING THE UNMODIFIED REFERENCE.
 
-TEST INFRASTRUCTURE ONLY (see oracle/README.md).  This script runs only in the build
-container, where /root/reference exists; the GPU box never runs it.  It imports the
-reference package from /root/reference (plus the logging shim oracle/shims/colortimelog),
+TEST INFRASTRUCTURE ONLY (see oracle/README.md).  This script runs only where a checkout of
+the reference exists (located as in oracle/build_ref.py); the tests never run it.  It imports the
+reference package from that checkout (plus the logging shim oracle/shims/colortimelog),
 trains the fixture models with the reference's own fit(), runs the reference's own
 predict_single() and, for a few utterances, drives the reference's own
 `_calculate_score` / `_update_beam_state` (uisrnn/uisrnn.py:388-477) step by step to record
@@ -37,7 +37,8 @@ import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(HERE)
-REF = '/root/reference'
+sys.path.insert(0, HERE)
+from build_ref import SOURCE as REF  # noqa: E402
 GOLD = os.path.join(REPO, 'tests', 'golden')
 CACHE = '/tmp/uis_golden_cache'
 
